@@ -1,9 +1,11 @@
 #!/usr/bin/env python
 """bench.py -- output pixels/s of UMPAModelDF.match() (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2] [--dump-outputs DIR]
 
-One "step" = one match() over one synthetic speckle stack of the named configuration.
+One "step" = one match() over one synthetic speckle stack of the named configuration; each GPU measurement below
+(value, e2e, stage times, gather) times K steps.  The stacks are generated from a fixed seed, so the same arguments
+give the same inputs on every run.
 N > 1 is launched with torchrun (one rank per GPU); the output rows of the SAME stack are
 split into N row bands (+ halo), no collective on the data path (strong scaling).
 
@@ -23,6 +25,9 @@ Printed JSON (one line, rank 0):
                computes anyway (tests/helpers.py::fp32_parity_stats).
   cpu_baseline the reference's own OpenMP CPU path (oracle/_ref, built from /root/reference) or
                the C port, timed on this box's host cores on a bounded ROI of the same workload.
+
+--dump-outputs DIR writes the maps the last timed step returned (see dump_outputs) so that two builds can be
+compared output for output.
 """
 import argparse
 import json
@@ -230,6 +235,24 @@ def reference_arm(args, cfg):
 
 # ------------------------------------------------------------------------------ our arm
 
+DUMP_SAMPLE_PX = 1 << 20
+
+
+def dump_outputs(out, directory, seed=0):
+    """Writes each map of one match_device() result as DIR/<name>.npy: float64 maps as float64, the integer maps (err,
+    debug_Ncalls) as float32, which holds them exactly.  A map of more than DUMP_SAMPLE_PX pixels is written as the
+    1-D sample np.sort(np.random.default_rng(seed).choice(pixels, DUMP_SAMPLE_PX, replace=False)) of its row-major
+    pixels, the same sample for every map: at most 2^20 x (5 x 8 + 2 x 4) bytes = 48 MiB in all."""
+    os.makedirs(directory, exist_ok=True)
+    maps = {k: v.cpu().numpy() for k, v in out.items() if not k.startswith("_")}     # (not the "_keepalive" entry)
+    n_px = next(iter(maps.values())).size
+    idx = None
+    if n_px > DUMP_SAMPLE_PX:
+        idx = np.sort(np.random.default_rng(seed).choice(n_px, DUMP_SAMPLE_PX, replace=False))
+    for k, v in maps.items():
+        v = v.astype(np.float64 if v.dtype == np.float64 else np.float32)
+        np.save(os.path.join(directory, k + ".npy"), v if idx is None else v.reshape(-1)[idx])
+
 STAGES = ("moments", "cross_table", "mean_table", "walk")
 
 
@@ -373,13 +396,15 @@ def ours(args, cfg):
     err_ok = None
     if rank == 0:
         err_ok = float((out["err"] == 1).sum().item()) / total_px          # rank 0 holds the whole map (gathered for N > 1)
+        if args.dump_outputs:
+            dump_outputs(out, args.dump_outputs)
 
     # ---- stage times of the kernels (events inside the library, same stream) -------
     stage_ms = None
     if sm.model is not None and info["path"] == "table":
         _capi.check(_capi.lib().umpa_set_profiling(sm.model._h, 1))
         acc = []
-        for _ in range(max(5, min(args.steps, 11))):
+        for _ in range(args.steps):
             sm.match_device(**kw)
             buf = (C.c_float * 4)()
             if _capi.lib().umpa_last_stage_ms(sm.model._h, buf, 4) == 4:
@@ -405,7 +430,7 @@ def ours(args, cfg):
         if "abc" in kw:
             kw_h["abc"] = kw["abc"][sm.band[0]:sm.band[1]].cpu().numpy()
         del sm, out
-        steps_e = max(2, min(args.steps, 10))
+        steps_e = args.steps
         d2h = 0
 
         stream_info = {}
@@ -576,7 +601,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the maps of the last timed step to DIR/<name>.npy (float32 / float64, a fixed seeded "
+                         "sample of 2^20 pixels of larger maps)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the maps of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = CONFIGS[args.config]
     if args.impl == "reference":

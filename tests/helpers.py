@@ -47,6 +47,22 @@ def roi_of(case):
     return tuple(tuple(int(v) for v in x) for x in r)
 
 
+def reference_matcher(kind, sam, ref, **model_kw):
+    """What a full-size parity test compares the product with: the UNMODIFIED reference (oracle/_ref) where its
+    compiled extension is present, otherwise the C restatement (oracle/port.py), which the golden vectors pin to the
+    reference.  The reference's sources are not part of this repository, so a plain checkout takes the restatement.
+    Returns (match(ROI, **kw) -> maps with the debug arrays fp32_parity_stats reads, name of the one used)."""
+    from oracle import port, ref as oref
+    R = oref.load()
+    threads = os.cpu_count()
+    if R is not None:
+        cls = {"NoDF": R.UMPAModelNoDF, "DF": R.UMPAModelDF, "DFKernel": R.UMPAModelDFKernel}[kind]
+        m = cls(list(sam), list(ref), **model_kw)
+        return (lambda ROI, **kw: m.match(ROI=ROI, num_threads=threads, quiet=True, **kw)), "reference"
+    om = port.OracleModel(kind, list(sam), list(ref), **model_kw)
+    return (lambda ROI, **kw: om.match(ROI=ROI, num_threads=threads, **kw)), "C restatement"
+
+
 def compare(got, exp, tol=1e-9, walk_exact=True, max_err_mismatch=0, max_outliers=0, outlier_tol=None,
             label=""):
     """Returns a dict of statistics; raises AssertionError with a readable message."""

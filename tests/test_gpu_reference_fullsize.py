@@ -1,8 +1,10 @@
 """GPU: the BASELINE.json configurations at FULL size against the UNMODIFIED reference (oracle/_ref, the
-reference's own C++/OpenMP model: UMPA/model.pyx:476-492 -> Model.cpp / Optim.cpp), directly.
+reference's own C++/OpenMP model: UMPA/model.pyx:476-492 -> Model.cpp / Optim.cpp), directly where its compiled
+extension is present, otherwise against the C restatement of it (oracle/port.py, pinned to the reference by the
+golden vectors): helpers.reference_matcher.
 
 The product matches the whole frame on the GPU (table path); the reference matches a block of rows of the SAME
-float64 stacks on the box's host cores (pixels are independent, so a block is exactly what the full run would
+float64 stacks on the host cores (pixels are independent, so a block is exactly what the full run would
 give there).  The blocks are placed across what the small golden fixtures cannot see: the edge of two row
 segments / chunks of the streaming table kernel, the edge of two column strips, the 2048- / 4096-wide pitch, S = 15.
 
@@ -15,12 +17,10 @@ import os
 import numpy as np
 import pytest
 
-from helpers import fp32_parity_stats
-from oracle import ref as oref
+from helpers import fp32_parity_stats, reference_matcher
 
 pytestmark = pytest.mark.gpu
 
-R = oref.load(build_if_missing=os.path.exists("/root/reference"))
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -51,14 +51,13 @@ def _run(kind, Na, N, Nw, ms, blocks, seed=2, abc_fn=None):
     from umpa_b200 import synth
     d = synth.speckle_stack(Na, N, N, seed=seed, max_shift=ms, dark_field=kind != "NoDF", device="cuda", as_numpy=False)
     cls = {"NoDF": umpa_b200.UMPAModelNoDF, "DF": umpa_b200.UMPAModelDF, "DFKernel": umpa_b200.UMPAModelDFKernel}[kind]
-    rcls = {"NoDF": R.UMPAModelNoDF, "DF": R.UMPAModelDF, "DFKernel": R.UMPAModelDFKernel}[kind]
     m = cls(list(d["sam"]), list(d["ref"]), window_size=Nw, max_shift=ms)
     kw = {}
     abc = None
     if kind == "DFKernel":
         abc = synth.blur_abc(*m.sh)
     sam_np, ref_np = d["sam"].cpu().numpy(), d["ref"].cpu().numpy()
-    rm = rcls([s for s in sam_np], [r for r in ref_np], window_size=Nw, max_shift=ms)
+    match_ref, against = reference_matcher(kind, sam_np, ref_np, window_size=Nw, max_shift=ms)
     merged = None
     for roi in blocks:
         (r0, r1, _), (c0, c1, _) = roi
@@ -66,7 +65,7 @@ def _run(kind, Na, N, Nw, ms, blocks, seed=2, abc_fn=None):
             kw["abc"] = np.ascontiguousarray(abc[r0:r1, c0:c1])
         got = m.match(ROI=roi, quiet=True, debug=False, **kw)
         assert m.last_match_info["path"] == "table", m.last_match_info
-        exp = rm.match(ROI=roi, num_threads=os.cpu_count(), quiet=True, **kw)
+        exp = match_ref(roi, **kw)
         st = fp32_parity_stats(got, exp)
         if merged is None:
             merged = st
@@ -78,15 +77,12 @@ def _run(kind, Na, N, Nw, ms, blocks, seed=2, abc_fn=None):
                     merged[k] += v
     merged["blocks"] = [list(map(list, b)) for b in blocks]
     merged["workload"] = "%s %dx%d^2 Nw=%d max_shift=%d" % (kind, Na, N, Nw, ms)
-    del m, rm, d
+    merged["against"] = against
+    del m, match_ref, d
     torch.cuda.empty_cache()
     return merged
 
 
-needs_ref = pytest.mark.skipif(R is None, reason="compiled reference (oracle/_ref) not available")
-
-
-@needs_ref
 def test_cfg2_block_vs_reference():
     """Config 2 (the metric): 96 full-width rows across the middle of the frame (where the streaming table kernel
     joins two row segments) and a 160-column block down the left edge over 600 rows (segment starts, chunk edges)."""
@@ -94,28 +90,24 @@ def test_cfg2_block_vs_reference():
     _check("cfg2", st)
 
 
-@needs_ref
 def test_cfg4_block_vs_reference():
     """Config 4 (DF 40 x 4096^2, Nw=3, max_shift=8, S=15): 64 rows through a tile edge, full width."""
     st = _run("DF", 40, 4096, 3, 8, [((2010, 2074, 1), (0, 4074, 1))])
     _check("cfg4", st)
 
 
-@needs_ref
 def test_cfg5_block_vs_reference():
     """Config 5 (NoDF 4 x 2048^2, Nw=6): 128 rows across the middle, full width."""
     st = _run("NoDF", 4, 2048, 6, 4, [((950, 1078, 1), (0, 2028, 1))])
     _check("cfg5", st, min_ok=.99)
 
 
-@needs_ref
 def test_cfg3_roi_vs_reference():
     """Config 3 (DFKernel 25 x 2048^2, Nw=3): a 48 x 48 ROI (the reference needs ~1 s per 2000 pixels here)."""
     st = _run("DFKernel", 25, 2048, 3, 5, [((1000, 1048, 1), (700, 748, 1))])
     _check("cfg3", st)
 
 
-@needs_ref
 def test_cfg1_full_vs_reference():
     """Config 1 (NoDF 10 x 256^2): the whole frame."""
     st = _run("NoDF", 10, 256, 2, 4, [((0, 244, 1), (0, 244, 1))])
