@@ -211,6 +211,62 @@ def fp32_parity_stats(got, exp, tol=1e-4, eps=3e-6, noise_floor=3e-6, max_probe=
     return st
 
 
+# ---------------------------------------------------------------------------------------------
+# Table costs entry by entry.  With sub_pixel_mode = 0 the walk leaves uv at its integer centre (walk_refine,
+# walk.cuh; Optim.cpp:399), so dy = c0 and dx = c1 exactly, and cell t of the 5x5 cache debug_d (-1: not evaluated)
+# holds the cost of the shift (si, sj) = (c0 + t // 5 - 2, c1 + t % 5 - 2).  A pixel that stopped with a bound error
+# (err == 0) has no reliable centre: locate_centre() finds it from the cached values.
+
+# |cost - cost64| <= COST_BOUND * (median FP64 cost of the case): the FP32 restatement of the table algebra meets it
+# (test_table_algebra.py), so a kernel that does not has another arithmetic, not other rounding
+COST_BOUND = 3e-5
+
+
+def cached_cells(res):
+    """(i, j, si, sj, cost) arrays of every cached cost of the err == 1 pixels of a sub_pixel_mode = 0 match."""
+    d, ok = np.asarray(res["debug_d"]), np.asarray(res["err"]) == 1
+    c0, c1 = np.asarray(res["dy"]), np.asarray(res["dx"])
+    assert np.array_equal(c0[ok], np.rint(c0[ok])) and np.array_equal(c1[ok], np.rint(c1[ok])), "non-integer centre"
+    i, j, t = np.nonzero(ok[:, :, None] & (d != -1))
+    return i, j, c0[i, j].astype(int) + t // 5 - 2, c1[i, j].astype(int) + t % 5 - 2, d[i, j, t]
+
+
+def locate_centre(d5, table, margin=100.):
+    """Centre (c0, c1) of a 5x5 walk cache whose centre is unknown: the offset at which its evaluated cells match the
+    pixel's (S, S) FP64 cost table best.  None when no cell was evaluated, or when another offset matches within a
+    factor `margin` as well (the match would be a guess)."""
+    d5 = np.asarray(d5)
+    t = np.nonzero(d5 != -1)[0]
+    h = (table.shape[0] - 1) // 2
+    if t.size == 0:
+        return None
+    devs = []
+    for c0 in range(-h - 2, h + 3):
+        for c1 in range(-h - 2, h + 3):
+            si, sj = c0 + t // 5 - 2, c1 + t % 5 - 2
+            if np.all(np.abs(si) <= h) and np.all(np.abs(sj) <= h):
+                devs.append((float(np.abs(d5[t] - table[si + h, sj + h]).max()), c0, c1))
+    devs.sort()
+    if not devs or (len(devs) > 1 and devs[1][0] <= margin * devs[0][0]):
+        return None
+    return devs[0][1], devs[0][2]
+
+
+def check_costs(got, exp, scale, label="", rows=None, bound=COST_BOUND):
+    """|got - exp| <= bound * scale for every cell; returns (max, 99.9th percentile) of |got - exp| / scale.
+    rows: the output row of every cell, named in the failure message."""
+    got, exp = np.asarray(got, np.float64), np.asarray(exp, np.float64)
+    assert got.size > 0, f"{label}: no cells compared"
+    r = np.abs(got - exp) / scale
+    r = np.where(np.isfinite(r), r, np.inf)
+    bad = r > bound
+    if bad.any():
+        where = "" if rows is None else ", rows %s" % sorted(set(int(v) for v in np.asarray(rows)[bad]))[:40]
+        raise AssertionError(f"{label}: {int(bad.sum())} of {r.size} costs off by more than {bound:g} of the cost "
+                             f"scale (max {r.max():.3g}{where})")
+    return float(r.max()), float(np.percentile(r, 99.9))
+
+
 def compare_fp32(got, exp, tol=1e-4, eps=3e-6, max_exception_frac=0.03, noise_floor=3e-6, label=""):
     """Parity check of the FP32 table path (tolerances of BASELINE.json north_star):
     err map and Ncalls (the integer walk) must be EQUAL; T, df within tol relative; dx, dy within

@@ -155,34 +155,52 @@ def test_bench_algorithmic_flops_match_survey():
     assert abs(e4 - 225 * ((40 + 7) * 32 / 24. + 7)) < 1e-9      # (Nw = 3: 24 of 32 columns are outputs)
 
 
-def test_table_plan_covers_every_supported_model():
+def test_table_plan_covers_every_supported_model(monkeypatch):
     """umpa_table_plan (plan_tiles, table_path.cu; host arithmetic): for every window / shift range / stack depth the
     table path accepts, the plan is one the kernel can run -- chunk height from the instantiated set, at least two ring
-    stages, the passes cover all S shift rows, the strips cover all columns, and pass-major streaming (order 2) only
-    where it is compiled (S >= 11) and needed (more than one pass)."""
+    stages, the passes cover all S shift rows, the strips cover all columns, pass-major streaming (order 2) only
+    where it is compiled (S >= 11) and needed (more than one pass), and a streaming chunk at least as high as its carry
+    (2 Nw rows: the next chunk's column pass reads all of them).  The same with 8-row chunks (two CTAs per SM,
+    UMPA_TAB_CTAS=2, or UMPA_TAB_EH=8): there Nw 5 and 6 have no plan (a halo tile of 8 rows holds no output row, a
+    streaming chunk of 8 rows is shorter than its carry), nor do some of the larger Nw 4 tables (shared memory), and
+    the planner says so instead of returning a plan."""
     import ctypes
     from umpa_b200 import _capi
     L = _capi.lib()
     out = (ctypes.c_int * 10)()
     seen = set()
-    for Nw in range(0, 7):
-        for ms in range(1, 11):
-            for Na in (1, 4, 25, 40, 120):
-                for rows, cols in ((1, 1), (37, 500), (254, 2034), (4074, 4074)):
-                    rc = L.umpa_table_plan(Na, Nw, ms, rows, cols, 148, out)
-                    assert rc == 0, (Nw, ms, Na, rows, cols, _capi.lib().umpa_last_error())
-                    EH, order, G, npass, FB, nstage, TW, nseg, nstrips, nt = list(out)
-                    S = 2 * ms - 1
-                    SH = 3 if S <= 9 else (2 if S <= 17 else 1)
-                    assert EH in (8, 16, 24, 32, 48) and order in (0, 1, 2)
-                    assert G >= 1 and npass >= 1 and npass * G * SH >= S and (npass - 1) * G * SH < S
-                    assert 1 <= FB <= Na and nstage >= 2
-                    assert TW == (32 - 2 * Nw) & ~3 and nstrips * TW >= cols > (nstrips - 1) * TW
-                    assert nseg >= 1 and nt == G * EH * 8 and nt <= 384
-                    if order == 2:
-                        assert S >= 11 and npass > 1
-                    if order == 0 and Nw > 0:
-                        assert EH - 2 * Nw >= 2
-                    seen.add(order)
-    assert seen == {0, 1, 2}
+    for ctas, eh in ((None, None), ("2", None), (None, "8"), ("2", "8")):
+        for name, v in (("UMPA_TAB_CTAS", ctas), ("UMPA_TAB_EH", eh)):
+            if v is None:
+                monkeypatch.delenv(name, raising=False)
+            else:
+                monkeypatch.setenv(name, v)
+        short = ctas is not None or eh is not None
+        env = (ctas, eh)
+        for Nw in range(0, 7):
+            for ms in range(1, 11):
+                for Na in (1, 4, 25, 40, 120):
+                    for rows, cols in ((1, 1), (37, 500), (254, 2034), (4074, 4074)):
+                        rc = L.umpa_table_plan(Na, Nw, ms, rows, cols, 148, out)
+                        if short and Nw >= 4 and rc != 0:
+                            assert rc == -4 and L.umpa_last_error().startswith(b"table path:"), (env, Nw, ms, rc)
+                            continue
+                        assert rc == 0, (env, Nw, ms, Na, rows, cols, L.umpa_last_error())
+                        assert not (short and Nw >= 5), (env, Nw, ms, list(out))
+                        EH, order, G, npass, FB, nstage, TW, nseg, nstrips, nt = list(out)
+                        S = 2 * ms - 1
+                        SH = 3 if S <= 9 else (2 if S <= 17 else 1)
+                        assert EH in ((8,) if short else (8, 16, 24, 32, 48)) and order in (0, 1, 2)
+                        assert G >= 1 and npass >= 1 and npass * G * SH >= S and (npass - 1) * G * SH < S
+                        assert 1 <= FB <= Na and nstage >= 2
+                        assert TW == (32 - 2 * Nw) & ~3 and nstrips * TW >= cols > (nstrips - 1) * TW
+                        assert nseg >= 1 and nt == G * EH * 8 and nt <= (192 if ctas else 384)
+                        if order == 2:
+                            assert S >= 11 and npass > 1
+                        if order == 0 and Nw > 0:
+                            assert EH - 2 * Nw >= 2
+                        if order in (1, 2):
+                            assert EH >= 2 * Nw, (env, Nw, ms, list(out))
+                        seen.add((short, order))
+    assert seen == {(s, o) for s in (False, True) for o in (0, 1, 2)}
     assert L.umpa_table_plan(25, 7, 5, 100, 100, 148, out) != 0          # Nw > 6 is not a table model

@@ -7,7 +7,7 @@ evaluation to rounding; in float32 it bounds the error the kernels can have."""
 import numpy as np
 import pytest
 
-from helpers import load_case
+from helpers import cached_cells, check_costs, load_case, locate_centre
 from oracle import port
 from table_algebra import cost_tables
 
@@ -135,3 +135,96 @@ def test_binary_shared_mask_is_the_unmasked_sums_minus_the_dead_window_positions
         (fo, to, vo), st = om.cost(i, j, si, sj)
         assert st == 1
         assert abs(f - fo) <= 1e-11 * abs(fo) and abs(t - to) <= 1e-11 * abs(to) and abs(v - vo) <= 1e-10 * max(1., abs(vo))
+
+
+MAPPING_CASES = [("DF", 2, 4, "sam"), ("NoDF", 1, 3, "sam"), ("NoDF", 0, 5, "sam"), ("NoDF", 0, 3, "ref"), ("DF", 1, 2, "sam"),
+                 ("DF", 2, 4, "ref"), ("NoDF", 1, 3, "ref"), ("DFKernel", 1, 3, "sam"), ("DFKernel", 2, 2, "ref")]
+
+
+def _oracle_match(kind, Nw, ms, assign, Na=6, H=40, W=44, seed=3):
+    from umpa_b200 import synth
+    Na = 26 if Nw == 0 else Na
+    pad = 8 if kind == "DFKernel" else 0
+    d = synth.speckle_stack(Na, H + 2 * pad, W + 2 * pad, seed=seed, max_shift=ms, dark_field=kind != "NoDF")
+    o = port.OracleModel(kind, list(d["sam"]), list(d["ref"]), window_size=Nw, max_shift=ms)
+    o.set_options(sub_pixel_mode=0, reference_shift=int(assign == "ref"))
+    N0, N1 = o.extent
+    abc = synth.blur_abc(N0, N1) if kind == "DFKernel" else None
+    return d, o, abc, o.match(abc=abc)
+
+
+@pytest.mark.parametrize("kind,Nw,ms,assign", MAPPING_CASES)
+def test_walk_cache_maps_to_shifts(kind, Nw, ms, assign):
+    """What tests/test_gpu_table_costs.py relies on to read the costs a match used: with sub_pixel_mode = 0 the
+    reference's walk returns its integer centre (dy, dx) = (c0, c1), and cell t of its 5x5 cache holds the cost of the
+    shift (c0 + t // 5 - 2, c1 + t % 5 - 2) -- the FP64 cost tables (assign_coordinates 'sam') or the direct cost
+    (any model).  max_shift 2: no pixel can complete its 4x4 block (err == 0), and locate_centre() finds the centre
+    from the cached values."""
+    d, o, abc, r = _oracle_match(kind, Nw, ms, assign)
+    h, p = ms - 1, o.padding
+    ok = r["err"] == 1
+    if ms == 2:
+        assert not ok.any()
+    else:
+        assert ok.mean() > .9
+    direct = kind == "DFKernel" or assign == "ref"
+    cost = lambda a, b, s, t: o.cost(p + a, p + b, s, t, () if abc is None else abc[a, b])[0][0]
+    if not direct:
+        c64, _, _ = cost_tables(d["sam"], d["ref"], Nw, ms, kind == "DF", np.float64)
+    if ms == 2:                                     # centres from the cached values
+        cells = []
+        for a, b in np.argwhere(~ok)[::8 if direct else 1]:
+            tab = c64[:, :, a, b] if not direct else np.array([[cost(a, b, s, t) for t in range(-h, h + 1)]
+                                                                for s in range(-h, h + 1)])
+            c = locate_centre(r["debug_d"][a, b], tab)
+            assert c is not None, (a, b)
+            cells += [(r["debug_d"][a, b, n], tab[c[0] + n // 5 - 2 + h, c[1] + n % 5 - 2 + h])
+                      for n in np.nonzero(r["debug_d"][a, b] != -1)[0]]
+        v, e = np.array(cells).T
+    else:
+        i, j, si, sj, v = cached_cells(r)
+        if not direct:
+            e = c64[si + h, sj + h, i, j]
+        else:
+            sel = np.arange(0, v.size, max(1, v.size // 400))    # the direct evaluation is slow for DFKernel
+            v = v[sel]
+            e = np.array([cost(*c) for c in zip(i[sel], j[sel], si[sel], sj[sel])])
+    scale = np.median(e)
+    assert v.size >= 100
+    np.testing.assert_array_less(np.abs(v - e), 1e-10 * scale)
+
+
+def test_cost_comparator_has_teeth(monkeypatch):
+    """check_costs (the FP64 comparison of tests/test_gpu_table_costs.py) on the cells a walk reads: it passes the FP32
+    restatement of the table algebra, and fails a table that lost one frame and one whose column filter reads one tap
+    a row too low."""
+    import table_algebra
+    kind, Nw, ms = "DF", 2, 4
+    d, o, _, r = _oracle_match(kind, Nw, ms, "sam", Na=11)
+    i, j, si, sj, v = cached_cells(r)
+    h = ms - 1
+    c64, _, _ = cost_tables(d["sam"], d["ref"], Nw, ms, True, np.float64)
+    scale = np.median(c64)
+    at = lambda c: c[si + h, sj + h, i, j]
+    c32, _, _ = cost_tables(d["sam"], d["ref"], Nw, ms, True, np.float32)
+    mx, _ = check_costs(at(c32), at(c64), scale, "float32 model")
+    assert mx > 0
+    dropped, _, _ = cost_tables(d["sam"][:-1], d["ref"][:-1], Nw, ms, True, np.float64)
+    with pytest.raises(AssertionError, match="costs off by"):
+        check_costs(at(dropped), at(c64), scale, "frame dropped")
+
+    def moved_tap(img, g, dtype):                   # table_algebra._filt, but column tap 0 reads row 1 instead of row 0
+        K = len(g)
+        H, W = img.shape[-2:]
+        tmp = np.zeros(img.shape[:-1] + (W - K + 1,), dtype=dtype)
+        for u in range(K):
+            tmp = (tmp + g[u] * img[..., :, u:u + W - K + 1]).astype(dtype)
+        out = np.zeros(img.shape[:-2] + (H - K + 1, W - K + 1), dtype=dtype)
+        for u in range(K):
+            r = u + (u == 0)
+            out = (out + g[u] * tmp[..., r:r + H - K + 1, :]).astype(dtype)
+        return out
+    monkeypatch.setattr(table_algebra, "_filt", moved_tap)
+    moved, _, _ = table_algebra.cost_tables(d["sam"], d["ref"], Nw, ms, True, np.float64)
+    with pytest.raises(AssertionError, match="costs off by"):
+        check_costs(at(moved), at(c64), scale, "tap moved")

@@ -656,6 +656,9 @@ size_t plan_tiles(TableParams &p, int S, bool filter, int *nt, int rows, int col
             if (e_eh ? atoi(e_eh) != eh : (eh == 8) != (ctas_sm > 1)) continue;     // 8-row chunks: two CTAs per SM only
             if (e_st && filter && halo > 0 && atoi(e_st) != stream) continue;
             if (!stream && eh - H2 < 2) continue;
+            // the carry of a chunk is its last 2*halo rows: a shorter chunk would leave carry rows unwritten that the
+            // next chunk's column pass reads (8-row chunks of UMPA_TAB_CTAS=2 / UMPA_TAB_EH=8 with Nw 5, 6)
+            if (stream && eh < H2) continue;
             TableParams q = p;
             q.EH = eh;
             q.G = std::min(max_nt / (eh * 8), (S + SH - 1) / SH);
@@ -734,7 +737,7 @@ extern "C" UMPA_API int umpa_table_plan(int Na, int Nw, int max_shift, int rows,
     p.Na = Na; p.Nw = Nw;
     int nt = 0;
     const size_t smem = plan_tiles(p, 2 * max_shift - 1, true, &nt, rows, cols, sm_count * ctas_per_sm(), ctas_per_sm());
-    if (!smem) { umpa_set_error("table path: tile does not fit shared memory"); return UMPA_ERR_UNSUPPORTED; }
+    if (!smem) { umpa_set_error("table path: no tile plan (shared memory, or chunks forced by UMPA_TAB_EH / UMPA_TAB_CTAS too short for the window)"); return UMPA_ERR_UNSUPPORTED; }
     const int v[10] = {p.EH, p.stream, p.G, p.npass, p.FB, p.nstage, p.TW, p.nseg, p.nstrips, nt};
     for (int i = 0; i < 10; i++) out[i] = v[i];
     return UMPA_OK;
@@ -888,7 +891,7 @@ static int table_match_impl(umpa_model *m, const RoiView &roi, const umpa_output
         const int ctas = m->sm_count * ctas_per_sm();
         smx = plan_tiles(px, S, true, &ntx, rows, cols + dxX, ctas, ctas_per_sm());
         smm = df ? plan_tiles(pm, S, false, &ntm, rows, cols + dxM, ctas, ctas_per_sm()) : 1;
-        if (!smx || !smm) { umpa_set_error("table path: tile does not fit shared memory"); return UMPA_ERR_UNSUPPORTED; }
+        if (!smx || !smm) { umpa_set_error("table path: no tile plan (shared memory, or chunks forced by UMPA_TAB_EH / UMPA_TAB_CTAS too short for the window)"); return UMPA_ERR_UNSUPPORTED; }
         const int rows_alloc = rows;
         int tpitch = px.cols_p;
         if (df) tpitch = std::max(tpitch, pm.cols_p);
