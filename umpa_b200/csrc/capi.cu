@@ -364,8 +364,16 @@ int zero_outputs(const umpa_outputs &o, size_t n, cudaStream_t st)
     return UMPA_OK;
 }
 
-// Centring constants of host frames, by host threads (hoststage.cu): the same values whether the
-// frames then go up in one piece, in bands, or partly converted.
+// Centring constant of host frame f (sample frames 0..Na-1, then reference frames; hoststage.cu): the same value
+// whether the frame then goes up in one piece, in bands, or partly converted.
+double host_frame_mean(const umpa_model *m, int f)
+{
+    const int k = f < m->Na ? f : f - m->Na, fh = m->dim[2 * k], fw = m->dim[2 * k + 1];
+    if (m->host_f32) return host_sampled_mean_f32(f < m->Na ? m->h_sam_f[k] : m->h_ref_f[k], fh, fw, table_row_step(fh));
+    return host_sampled_mean(f < m->Na ? m->h_sam[k] : m->h_ref[k], fh, fw, table_row_step(fh));
+}
+
+// the constants of all 2 Na frames, by host threads
 void host_means(const umpa_model *m, std::vector<double> &mu)
 {
     const int Na = m->Na;
@@ -375,9 +383,7 @@ void host_means(const umpa_model *m, std::vector<double> &mu)
         for (;;) {
             const int f = next.fetch_add(1);
             if (f >= 2 * Na) break;
-            const int k = f < Na ? f : f - Na, fh = m->dim[2 * k], fw = m->dim[2 * k + 1];
-            if (m->host_f32) mu[f] = host_sampled_mean_f32(f < Na ? m->h_sam_f[k] : m->h_ref_f[k], fh, fw, table_row_step(fh));
-            else mu[f] = host_sampled_mean(f < Na ? m->h_sam[k] : m->h_ref[k], fh, fw, table_row_step(fh));
+            mu[f] = host_frame_mean(m, f);
         }
     };
     size_t samples = 0;                          // what the threads share: small jobs are not worth a thread start
@@ -603,6 +609,41 @@ bool same_allocation(const void *lo, const void *hi)
     return (unsigned long long)(uintptr_t)hi <= base + size;
 }
 
+// Byte distance between consecutive host frames (frame_bytes each) when they are equally spaced, without overlap,
+// inside ONE pinned allocation -- a 2-D copy must not span two -- and 0 otherwise.
+size_t frame_spacing(const std::vector<const void *> &f, size_t frame_bytes)
+{
+    if (f.size() < 2) return frame_bytes;
+    const ptrdiff_t d = (const char *)f[1] - (const char *)f[0];
+    if (d < (ptrdiff_t)frame_bytes) return 0;
+    for (size_t k = 2; k < f.size(); k++)
+        if ((const char *)f[k] - (const char *)f[k - 1] != d) return 0;
+    return same_allocation(f[0], (const char *)f.back() + frame_bytes) ? (size_t)d : 0;
+}
+
+// Host -> device copy, on `st`, of rows [y0, y1) of Na frames, `width` bytes of each row.  Host frame k starts at
+// src[k], or at src[0] + k * sstride when the frames lie in one pinned block (sstride > 0, see frame_spacing); it holds
+// rows sy, sy + 1, ... spitch bytes apart.  Device frame k starts at dst + k * dstride, rows dpitch bytes apart.
+// One 2-D copy covers all frames when the source is one block, the rows are contiguous on both sides and both strides
+// are legal cudaMemcpy2D pitches (cudaDevAttrMaxPitch = 2^31 - 1 bytes); otherwise one copy per frame, a 2-D one
+// when the rows are not contiguous.
+cudaError_t upload_rows(void *dst, size_t dstride, size_t dpitch, const void *const *src, size_t sstride, size_t spitch,
+                        int sy, size_t width, int Na, int y0, int y1, cudaStream_t st)
+{
+    const size_t max_pitch = ((size_t)1 << 31) - 1, rows = (size_t)(y1 - y0), soff = (size_t)(y0 - sy) * spitch;
+    const bool packed = spitch == width && dpitch == width;
+    char *d = (char *)dst + (size_t)y0 * dpitch;
+    if (sstride > 0 && packed && sstride <= max_pitch && dstride <= max_pitch)
+        return cudaMemcpy2DAsync(d, dstride, (const char *)src[0] + soff, sstride, rows * width, Na, cudaMemcpyHostToDevice, st);
+    for (int k = 0; k < Na; k++, d += dstride) {
+        const char *s = (sstride > 0 ? (const char *)src[0] + k * sstride : (const char *)src[k]) + soff;
+        const cudaError_t e = packed ? cudaMemcpyAsync(d, s, rows * width, cudaMemcpyHostToDevice, st)
+                                     : cudaMemcpy2DAsync(d, dpitch, s, spitch, width, rows, cudaMemcpyHostToDevice, st);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
 int host_threads()
 {
     if (const char *e = getenv("UMPA_HOST_THREADS")) return std::max(0, atoi(e));
@@ -613,15 +654,6 @@ int host_threads()
     return std::max(0, std::min(12, hw / ranks - (ranks > 1 ? 2 : 4)));
 }
 
-// The pipelined host-to-host match.  Frames still in host memory go up in row bands on a copy stream
-// while the kernels of the previous band run and the maps of the band before that go back to the host.
-// Band b needs input rows below off0 + step0*(r1-1) + padding only, so its kernels start as soon as
-// those rows have landed.  PCIe is the critical path (1.68 GB of FP64 for config 2 against ~4 ms of
-// kernels), so host threads shorten it: they take the centring constants from the sampled rows and
-// convert the LOWER part of every frame to centred FP32 in pinned staging (same arithmetic as
-// center_frames: FP64 subtract, one rounding) while the DMA engine is busy with the upper part in
-// FP64; the converted rows then cross at half the bytes, straight into the FP32 stacks.
-// Pixels are independent: the result is the one the unpipelined path gives for the same constants.
 // Row bands of a pipelined match: equal slices of the N0 output rows, the last one halved twice so that little
 // work is left when the final rows arrive (kernels and download hide behind the upload).  UMPA_BANDS overrides.
 std::vector<int> band_edges(int N0)
@@ -640,90 +672,100 @@ std::vector<int> band_edges(int N0)
     return edge;
 }
 
-int streamed_match_f32(umpa_model *m, const RoiView &v, const umpa_outputs &dev, const umpa_outputs &host);
-
+// The pipelined host-to-host match.  Frames still in host memory go up in row bands on a copy stream
+// while the kernels of the previous band run and the maps of the band before that go back to the host.
+// Band b needs input rows below off0 + step0*(r1-1) + padding only, so its kernels start as soon as
+// those rows have landed.  Each band's new rows arrive in two parts, split at row Yc of every frame:
+//  * direct rows (< Yc) cross PCIe in the frames' own element type.  Float64 rows land in the FP64 stacks
+//    and are centred into the FP32 stacks (center_frames); float32 rows, half the bytes, land in the FP32
+//    stacks and are centred where they lie (center_inplace).
+//  * staged rows (>= Yc) are centred to FP32 by host threads into pinned staging (same arithmetic as
+//    center_frames: FP64 subtract, one rounding) while the DMA engine is busy with the direct rows, and
+//    then cross at FP32 size straight into the FP32 stacks.
+// PCIe is the critical path (1.68 GB of FP64 for config 2 against ~4 ms of kernels), so for float64 frames
+// the host threads shorten it by staging the lower rows; they also take the centring constants from the
+// sampled rows.
+// Pixels are independent: the result is the one the unpipelined path gives for the same constants.
 int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, const umpa_outputs &host)
 {
     const int Na = m->Na, H = m->H, W = m->W, pitch = m->pitch;
+    const bool f32 = m->host_f32;
     const std::vector<int> edge = band_edges(v.N0);     // band b = output rows [edge[b], edge[b+1])
     const int nb = (int)edge.size() - 1;
     std::vector<int> need(nb);                  // band b needs input rows [0, need[b])
     for (int b = 0; b < nb; b++)
         need[b] = b == nb - 1 ? H : std::min(H, v.off0 + v.step0 * (edge[b + 1] - 1) + m->padding + 1);
 
-    // host conversion: rows [Yc, H) of every frame are converted by nthr host threads
+    // direct rows: host stacks (sample, reference) -> FP64 stacks (float64 frames) or FP32 stacks (float32 frames)
+    std::vector<const void *> src[2];
+    if (f32) { src[0].assign(m->h_sam_f.begin(), m->h_sam_f.end()); src[1].assign(m->h_ref_f.begin(), m->h_ref_f.end()); }
+    else { src[0].assign(m->h_sam.begin(), m->h_sam.end()); src[1].assign(m->h_ref.begin(), m->h_ref.end()); }
+    void *const ddst[2] = {f32 ? (void *)m->d_sam32 : m->d_sam64, f32 ? (void *)m->d_ref32 : m->d_ref64};
+    const size_t rowb = (size_t)W * (f32 ? sizeof(float) : sizeof(double));    // bytes of a host row
+    const size_t drow = f32 ? (size_t)pitch * sizeof(float) : rowb;            // ... and of its device row
+    const size_t srow = (size_t)pitch * sizeof(float);                          // a staged row, on both sides
+    const size_t sstride[2] = {frame_spacing(src[0], (size_t)H * rowb), frame_spacing(src[1], (size_t)H * rowb)};
+    cudaPointerAttributes pa{};
+    const bool pinned = cudaPointerGetAttributes(&pa, src[0][0]) == cudaSuccess && pa.type != cudaMemoryTypeUnregistered;
+    cudaGetLastError();
+
+    // route: nthr host threads stage rows [Yc, H) of every frame.  Pageable frames would crawl through the driver's
+    // own staging (measured: 80 ms for config 2 in float32), so the host stages all of their rows.
     int nthr = nb > 1 ? host_threads() : 0;
     int Yc = H;
-    if (m->host_f32) {
-        // float32 frames: pinned ones go up as they are at the full DMA rate (streamed_match_f32); pageable ones
-        // would crawl through the driver's staging (measured: 80 ms for config 2), so the host threads centre ALL
-        // their rows into the pinned staging instead -- the float64 machinery below with a float source.
-        cudaPointerAttributes pa{};
-        const bool pinned = cudaPointerGetAttributes(&pa, m->h_sam_f[0]) == cudaSuccess && pa.type != cudaMemoryTypeUnregistered;
-        cudaGetLastError();
-        if (pinned || nthr == 0) return streamed_match_f32(m, v, dev, host);
-        Yc = 0;
-    } else if (nthr > 0) {
-        // Which share x of the rows should the host convert?  Per input byte a converted row costs the
-        // host memory system 2 bytes of traffic (read, write FP32, DMA read of the FP32) against 1 for a
-        // row that goes up as FP64, and PCIe half a byte against one.  With M = B_conc + 1.5 R_conc the
-        // memory bandwidth this process got while both sides ran, and B_alone the DMA rate with nobody
-        // converting:   PCIe time (1 - x/2) D / B_alone  ==  memory time (1 + x) D / M
-        //           =>  x = (M - B_alone) / (M/2 + B_alone).
-        // On an idle host (B_conc = B_alone = B) this is the CPU balance x = 1 / (B/R + 1/2); when several
-        // ranks saturate the host memory (measured: 2 ranks on one 24-vCPU box, DMA 53 -> 40 GB/s,
-        // conversion 73 -> 36 GB/s) it backs off, down to plain DMA.
-        cudaPointerAttributes pa{};
-        const bool pinned = cudaPointerGetAttributes(&pa, m->h_sam[0]) == cudaSuccess && pa.type != cudaMemoryTypeUnregistered;
-        cudaGetLastError();
-        double Ba, Bc, Rc;
-        {
-            std::lock_guard<std::mutex> lk(g_rates.mu);
-            if (pinned && g_rates.dma_alone_gbs == 0.) {       // once per process: ~128 MB of real rows, nobody converting
-                const int pr = std::max(1, std::min(H, (int)(((size_t)128 << 20) / ((size_t)Na * W * sizeof(double)))));
-                const size_t bytes = (size_t)pr * W * sizeof(double);
-                ptrdiff_t gap = Na > 1 ? m->h_sam[1] - m->h_sam[0] : (ptrdiff_t)H * W;
-                for (int k = 2; k < Na; k++) if (m->h_sam[k] - m->h_sam[k - 1] != gap) gap = 0;
-                if (gap > 0 && !same_allocation(m->h_sam[0], m->h_sam[Na - 1] + (size_t)H * W)) gap = 0;
-                cudaEvent_t e0 = nullptr, e1 = nullptr;
-                cudaEventCreate(&e0); cudaEventCreate(&e1);
-                cudaEventRecord(e0, m->s_copy);
-                if (gap >= (ptrdiff_t)H * W && gap * (ptrdiff_t)sizeof(double) < ((ptrdiff_t)1 << 31))
-                    cudaMemcpy2DAsync(m->d_sam64, (size_t)H * W * sizeof(double), m->h_sam[0], (size_t)gap * sizeof(double), bytes, Na,
-                                      cudaMemcpyHostToDevice, m->s_copy);
-                else
-                    for (int k = 0; k < Na; k++)
-                        cudaMemcpyAsync(m->d_sam64 + m->frame_off[k], m->h_sam[k], bytes, cudaMemcpyHostToDevice, m->s_copy);
-                cudaEventRecord(e1, m->s_copy);
-                float ms = 0.f;
-                if (cudaEventSynchronize(e1) == cudaSuccess && cudaEventElapsedTime(&ms, e0, e1) == cudaSuccess && ms > 0.f)
-                    g_rates.dma_alone_gbs = (double)Na * bytes / (ms * 1e-3) / 1e9;
-                cudaEventDestroy(e0); cudaEventDestroy(e1);
-                cudaGetLastError();
+    if (nthr > 0) {
+        double x;                                       // share of the rows the host stages
+        if (f32) {
+            x = pinned ? 0. : 1.;                       // pinned float32 rows go up as they are, at the full DMA rate
+        } else {
+            // Which share x of the rows should the host convert?  Per input byte a converted row costs the
+            // host memory system 2 bytes of traffic (read, write FP32, DMA read of the FP32) against 1 for a
+            // row that goes up as FP64, and PCIe half a byte against one.  With M = B_conc + 1.5 R_conc the
+            // memory bandwidth this process got while both sides ran, and B_alone the DMA rate with nobody
+            // converting:   PCIe time (1 - x/2) D / B_alone  ==  memory time (1 + x) D / M
+            //           =>  x = (M - B_alone) / (M/2 + B_alone).
+            // On an idle host (B_conc = B_alone = B) this is the CPU balance x = 1 / (B/R + 1/2); when several
+            // ranks saturate the host memory (measured: 2 ranks on one 24-vCPU box, DMA 53 -> 40 GB/s,
+            // conversion 73 -> 36 GB/s) it backs off, down to plain DMA.
+            double Ba, Bc, Rc;
+            {
+                std::lock_guard<std::mutex> lk(g_rates.mu);
+                if (pinned && g_rates.dma_alone_gbs == 0.) {       // once per process: ~128 MB of real rows, nobody converting
+                    const int pr = std::max(1, std::min(H, (int)(((size_t)128 << 20) / ((size_t)Na * rowb))));
+                    cudaEvent_t e0 = nullptr, e1 = nullptr;
+                    cudaEventCreate(&e0); cudaEventCreate(&e1);
+                    cudaEventRecord(e0, m->s_copy);
+                    upload_rows(m->d_sam64, (size_t)H * rowb, rowb, src[0].data(), sstride[0], rowb, 0, rowb, Na, 0, pr, m->s_copy);
+                    cudaEventRecord(e1, m->s_copy);
+                    float ms = 0.f;
+                    if (cudaEventSynchronize(e1) == cudaSuccess && cudaEventElapsedTime(&ms, e0, e1) == cudaSuccess && ms > 0.f)
+                        g_rates.dma_alone_gbs = (double)Na * pr * rowb / (ms * 1e-3) / 1e9;
+                    cudaEventDestroy(e0); cudaEventDestroy(e1);
+                    cudaGetLastError();
+                }
+                Ba = g_rates.dma_alone_gbs > 0. ? g_rates.dma_alone_gbs : 55.;
+                Bc = g_rates.dma_gbs > 0. ? g_rates.dma_gbs : Ba;
+                Rc = g_rates.conv_gbs > 0. ? g_rates.conv_gbs : std::min(85., 6.5 * nthr);
             }
-            Ba = g_rates.dma_alone_gbs > 0. ? g_rates.dma_alone_gbs : 55.;
-            Bc = g_rates.dma_gbs > 0. ? g_rates.dma_gbs : Ba;
-            Rc = g_rates.conv_gbs > 0. ? g_rates.conv_gbs : std::min(85., 6.5 * nthr);
+            const double Mem = Bc + 1.5 * Rc;
+            x = (Mem - Ba) / (.5 * Mem + Ba);
+            if (x < .15) x = 0.;                               // not worth the threads
+            x = std::min(x, .9);
+            if (!pinned) x = 1.;
+            if (const char *e = getenv("UMPA_HOST_FRAC")) x = atof(e);
+            x = std::max(0., std::min(1., x));
         }
-        const double Mem = Bc + 1.5 * Rc;
-        double x = (Mem - Ba) / (.5 * Mem + Ba);
-        if (x < .15) x = 0.;                               // not worth the threads
-        x = std::min(x, .9);
-        // pageable frames go through the driver's own staging at a fraction of the pinned rate: convert everything
-        if (!pinned) x = 1.;
-        if (const char *e = getenv("UMPA_HOST_FRAC")) x = atof(e);
-        x = std::max(0., std::min(1., x));
         Yc = H - (int)(x * H);
         if (Yc >= H) nthr = 0;
     }
-    int HC = H - Yc;                            // converted rows per frame
+    int HC = H - Yc;                            // staged rows per frame
     std::unique_lock<std::mutex> stage_lock(g_stage.mu, std::defer_lock);
     if (nthr > 0) {
         stage_lock.lock();
-        const size_t want = (size_t)2 * Na * HC * pitch * sizeof(float);
+        const size_t want = (size_t)2 * Na * HC * srow;
         if (g_stage.bytes < want) {
-            // room for every split the rate model may pick later (all rows when the frames are pageable or float32)
-            const size_t want_max = (size_t)2 * Na * H * pitch * sizeof(float);
+            // room for every split the rate model may pick later (all rows when the frames are pageable)
+            const size_t want_max = (size_t)2 * Na * H * srow;
             if (getenv("UMPA_STAGE_SYNC")) {
                 stage_release_locked();
                 if (cudaHostAlloc((void **)&g_stage.p, want_max, cudaHostAllocDefault) == cudaSuccess) g_stage.bytes = want_max;
@@ -737,26 +779,11 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
             stage_lock.unlock();
         }
     }
-    if (m->host_f32 && nthr == 0) return streamed_match_f32(m, v, dev, host);    // no staging: plain copies after all
 
-    // frames that are equally spaced slices of one host stack go up with one 2-D copy per stack and band
-    // (cudaMemcpy2D pitches are limited to cudaDevAttrMaxPitch = 2^31 - 1 bytes, and the whole source range has
-    //  to lie inside ONE pinned allocation: equally spaced frames from separate allocations are rejected)
-    const ptrdiff_t max_pitch = ((ptrdiff_t)1 << 31) - 1;
-    auto spacing = [&](const std::vector<const double *> &h) -> ptrdiff_t {
-        if ((ptrdiff_t)H * W * (ptrdiff_t)sizeof(double) > max_pitch) return 0;
-        if (Na < 2) return (ptrdiff_t)H * W;
-        const ptrdiff_t d = h[1] - h[0];
-        if (d < (ptrdiff_t)H * W || d * (ptrdiff_t)sizeof(double) > max_pitch) return 0;
-        for (int k = 2; k < Na; k++) if (h[k] - h[k - 1] != d) return 0;
-        return same_allocation(h[0], h[Na - 1] + (size_t)H * W) ? d : 0;
-    };
-    const ptrdiff_t gap_s = m->host_f32 ? 0 : spacing(m->h_sam), gap_r = m->host_f32 ? 0 : spacing(m->h_ref);
-
-    // ---- host workers: constants first, then conversion jobs in the order the bands need them ----
+    // ---- host workers: constants first, then staging jobs in the order the bands need them ----
     struct Job { int band, stack, frame, y0, y1; };
     std::vector<Job> jobs;
-    std::vector<int> cy0(nb, 0), cy1(nb, 0);    // converted rows that band b waits for: [cy0, cy1)
+    std::vector<int> cy0(nb, 0), cy1(nb, 0);    // staged rows that band b waits for: [cy0, cy1)
     {
         int hi = Yc;
         for (int b = 0; b < nb && nthr > 0; b++) {
@@ -773,13 +800,11 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
     std::atomic<bool> abort_flag{false};
     using clk = std::chrono::steady_clock;
     std::vector<clk::time_point> conv_t0(std::max(nthr, 1)), conv_t1(std::max(nthr, 1));
-    const int rs = table_row_step(H);
     auto worker = [&](int wid) {
         for (;;) {
             const int f = next_mean.fetch_add(1);
             if (f >= 2 * Na) break;
-            if (m->host_f32) mu[f] = host_sampled_mean_f32(f < Na ? m->h_sam_f[f] : m->h_ref_f[f - Na], H, W, rs);
-            else mu[f] = host_sampled_mean(f < Na ? m->h_sam[f] : m->h_ref[f - Na], H, W, rs);
+            mu[f] = host_frame_mean(m, f);
         }
         means_done.fetch_add(1, std::memory_order_acq_rel);
         while (means_done.load(std::memory_order_acquire) < nthr) std::this_thread::yield();
@@ -789,11 +814,10 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
             if (j >= (int)jobs.size() || abort_flag.load()) break;
             const Job &q = jobs[j];
             float *dst = g_stage.p + ((size_t)(q.stack * Na + q.frame) * HC + (q.y0 - Yc)) * pitch;
-            const double c = mu[q.stack == 0 ? q.frame : Na + q.frame];
-            if (m->host_f32)
-                host_center_rows_f32(dst, (q.stack == 0 ? m->h_sam_f[q.frame] : m->h_ref_f[q.frame]) + (size_t)q.y0 * W, q.y1 - q.y0, W, pitch, c);
-            else
-                host_center_rows(dst, (q.stack == 0 ? m->h_sam[q.frame] : m->h_ref[q.frame]) + (size_t)q.y0 * W, q.y1 - q.y0, W, pitch, c);
+            const double c = mu[q.stack * Na + q.frame];
+            const void *s = src[q.stack][q.frame];
+            if (f32) host_center_rows_f32(dst, (const float *)s + (size_t)q.y0 * W, q.y1 - q.y0, W, pitch, c);
+            else host_center_rows(dst, (const double *)s + (size_t)q.y0 * W, q.y1 - q.y0, W, pitch, c);
             left[q.band].fetch_sub(1, std::memory_order_acq_rel);
             conv_t1[wid] = clk::now();
         }
@@ -801,7 +825,7 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
     std::vector<std::thread> pool;
     for (int t = 0; t < nthr; t++) pool.emplace_back(worker, t);
 
-    std::vector<cudaEvent_t> ev(2 * nb + 1, nullptr);
+    std::vector<cudaEvent_t> ev(2 * nb, nullptr);
     cudaEvent_t rate_ev[2] = {nullptr, nullptr}; // around the first band's FP64 rows: the DMA rate
     int rc = UMPA_OK;
     auto fail = [&](int code) {
@@ -814,9 +838,9 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
     };
 #define ST_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
         umpa_set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); return fail(UMPA_ERR_CUDA); } } while (0)
+    for (auto &e : ev) ST_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     const bool trace = getenv("UMPA_STREAM_TRACE") != nullptr;     // timeline of the three streams on stderr
-    for (auto &e : ev) ST_CUDA(cudaEventCreateWithFlags(&e, trace ? cudaEventDefault : cudaEventDisableTiming));
-    std::vector<cudaEvent_t> tev;                // trace only: [start, constants, then per band: copy, comp, out]
+    std::vector<cudaEvent_t> tev;                // trace only: start, then per band: copy, comp, out
     auto mark = [&](cudaStream_t st) {
         if (!trace) return;
         cudaEvent_t e = nullptr;
@@ -827,36 +851,6 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
     if (trace) { cudaStreamSynchronize(m->s_copy); cudaStreamSynchronize(m->s_comp); }
     mark(m->s_copy);
 
-    const size_t rowb = (size_t)W * sizeof(double);
-    // FP64 rows [y0, y1) of every frame of one stack -> FP64 device stack
-    auto upload64 = [&](double *dst, const std::vector<const double *> &h, ptrdiff_t gap, int y0, int y1) -> cudaError_t {
-        const size_t bytes = (size_t)(y1 - y0) * rowb;
-        if (gap > 0)
-            return cudaMemcpy2DAsync(dst + (size_t)y0 * W, (size_t)H * rowb, h[0] + (size_t)y0 * W, (size_t)gap * sizeof(double),
-                                     bytes, Na, cudaMemcpyHostToDevice, m->s_copy);
-        for (int k = 0; k < Na; k++) {
-            cudaError_t e = cudaMemcpyAsync(dst + m->frame_off[k] + (size_t)y0 * W, h[k] + (size_t)y0 * W, bytes,
-                                            cudaMemcpyHostToDevice, m->s_copy);
-            if (e != cudaSuccess) return e;
-        }
-        return cudaSuccess;
-    };
-    // converted rows [y0, y1) (>= Yc) of every frame of one stack: staging -> centred FP32 device stack
-    auto upload32 = [&](float *dst, int stack, int y0, int y1) -> cudaError_t {
-        const size_t rb = (size_t)pitch * sizeof(float);
-        const float *src = g_stage.p + ((size_t)stack * Na * HC + (y0 - Yc)) * pitch;
-        if ((ptrdiff_t)((size_t)H * rb) <= max_pitch)
-            return cudaMemcpy2DAsync(dst + (size_t)y0 * pitch, (size_t)H * rb, src, (size_t)HC * rb, (size_t)(y1 - y0) * rb, Na,
-                                     cudaMemcpyHostToDevice, m->s_copy);
-        for (int k = 0; k < Na; k++) {
-            cudaError_t e = cudaMemcpyAsync(dst + ((size_t)k * H + y0) * pitch, src + (size_t)k * HC * pitch, (size_t)(y1 - y0) * rb,
-                                            cudaMemcpyHostToDevice, m->s_copy);
-            if (e != cudaSuccess) return e;
-        }
-        return cudaSuccess;
-    };
-
-    mark(m->s_copy);
     size_t rate_bytes = 0;
     if (nthr > 0) { cudaEventCreate(&rate_ev[0]); cudaEventCreate(&rate_ev[1]); cudaEventRecord(rate_ev[0], m->s_copy); }
     int up_hi = 0;                              // rows [0, up_hi) are on the device and centred
@@ -865,27 +859,31 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
     for (int b = 0; b < nb; b++) {
         const int r0 = edge[b], r1 = edge[b + 1];
         const int hi = std::max(up_hi, need[b]);
-        const int d1 = std::min(hi, Yc);         // FP64 part [up_hi, d1), converted part [max(up_hi, Yc), hi)
+        const int d1 = std::min(hi, Yc), s0 = std::max(up_hi, Yc);     // direct rows [up_hi, d1), staged rows [s0, hi)
         if (d1 > up_hi) {
-            ST_CUDA(upload64(m->d_sam64, m->h_sam, gap_s, up_hi, d1));
-            ST_CUDA(upload64(m->d_ref64, m->h_ref, gap_r, up_hi, d1));
+            for (int a = 0; a < 2; a++)
+                ST_CUDA(upload_rows(ddst[a], (size_t)H * drow, drow, src[a].data(), sstride[a], rowb, 0, rowb, Na, up_hi, d1, m->s_copy));
             if (b == 0 && rate_ev[1]) { cudaEventRecord(rate_ev[1], m->s_copy); rate_bytes = (size_t)2 * Na * (d1 - up_hi) * rowb; }
         }
-        if (!have_means) {                       // the first FP64 rows are on their way; now the constants
+        if (!have_means) {                       // the first direct rows are on their way; now the constants
             if (nthr > 0) while (means_done.load(std::memory_order_acquire) < nthr) std::this_thread::yield();
             else host_means(m, mu);
             if ((rc = table_set_means(m, mu.data(), m->s_comp))) return fail(rc);
             have_means = true;
         }
-        if (hi > std::max(up_hi, Yc)) {
+        if (hi > s0) {
             while (left[b].load(std::memory_order_acquire) > 0) std::this_thread::yield();
-            ST_CUDA(upload32(m->d_sam32, 0, std::max(up_hi, Yc), hi));
-            ST_CUDA(upload32(m->d_ref32, 1, std::max(up_hi, Yc), hi));
+            for (int a = 0; a < 2; a++) {
+                const void *stage = g_stage.p + (size_t)a * Na * HC * pitch;     // stack a: frame k holds rows [Yc, H)
+                ST_CUDA(upload_rows(a ? m->d_ref32 : m->d_sam32, (size_t)H * srow, srow, &stage, (size_t)HC * srow, srow, Yc, srow,
+                                    Na, s0, hi, m->s_copy));
+            }
         }
         ST_CUDA(cudaEventRecord(ev[2 * b], m->s_copy));
         mark(m->s_copy);
         ST_CUDA(cudaStreamWaitEvent(m->s_comp, ev[2 * b], 0));
-        if ((rc = table_center_rows(m, up_hi, std::max(up_hi, d1), m->s_comp))) return fail(rc);
+        const int c1 = std::max(up_hi, d1);
+        if ((rc = f32 ? table_center_rows_inplace(m, up_hi, c1, m->s_comp) : table_center_rows(m, up_hi, c1, m->s_comp))) return fail(rc);
         up_hi = hi;
         RoiView vb = v;
         vb.off0 = v.off0 + v.step0 * r0; vb.N0 = r1 - r0;
@@ -910,22 +908,21 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
     ST_CUDA(cudaStreamSynchronize(m->s_copy));
 #undef ST_CUDA
     if (trace) {
-        float t = 0.f;
-        cudaEventElapsedTime(&t, tev[0], tev[1]);
-        fprintf(stderr, "[umpa stream] %d bands, %d host threads convert rows >= %d of %d; sampled rows up at %.2f ms\n", nb, nthr, Yc, H, t);
+        fprintf(stderr, "[umpa stream] %s frames, %d bands, %d host threads stage rows >= %d of %d\n",
+                f32 ? "float32" : "float64", nb, nthr, Yc, H);
         for (int b = 0; b < nb; b++) {
             float tc = 0.f, tk = 0.f, to = 0.f;
-            cudaEventElapsedTime(&tc, tev[0], tev[2 + 3 * b]);
-            cudaEventElapsedTime(&tk, tev[0], tev[3 + 3 * b]);
-            cudaEventElapsedTime(&to, tev[0], tev[4 + 3 * b]);
+            cudaEventElapsedTime(&tc, tev[0], tev[1 + 3 * b]);
+            cudaEventElapsedTime(&tk, tev[0], tev[2 + 3 * b]);
+            cudaEventElapsedTime(&to, tev[0], tev[3 + 3 * b]);
             fprintf(stderr, "[umpa stream] band %2d: uploaded %.2f  computed %.2f  downloaded %.2f ms\n", b, tc, tk, to);
         }
         for (auto e : tev) cudaEventDestroy(e);
     }
     for (auto e : ev) if (e) cudaEventDestroy(e);
     m->host_pending = false;
-    m->fp64_missing = Yc < H;
-    if (nthr > 0 && !jobs.empty() && !m->host_f32) {     // update the measured rates
+    m->fp64_missing = f32 || Yc < H;            // no FP64 copy of these rows on the device: ensure_resident makes one on demand
+    if (nthr > 0 && !jobs.empty() && !f32) {    // update the measured rates
         clk::time_point a = conv_t0[0], z = conv_t1[0];
         for (int t = 1; t < nthr; t++) { a = std::min(a, conv_t0[t]); z = std::max(z, conv_t1[t]); }
         const double secs = std::chrono::duration<double>(z - a).count();
@@ -941,114 +938,6 @@ int streamed_match(umpa_model *m, const RoiView &v, const umpa_outputs &dev, con
     }
     for (auto e : rate_ev) if (e) cudaEventDestroy(e);
     m->stream_bands = nb; m->stream_threads = nthr; m->stream_host_rows = HC;
-    return UMPA_OK;
-}
-
-// The same pipeline for float32 host frames (umpa_set_frames_f32): the rows cross PCIe as they are -- half
-// the bytes of the float64 route, so no host conversion -- straight into the FP32 stacks, and are centred there.
-int streamed_match_f32(umpa_model *m, const RoiView &v, const umpa_outputs &dev, const umpa_outputs &host)
-{
-    const int Na = m->Na, H = m->H, W = m->W, pitch = m->pitch;
-    const std::vector<int> edge = band_edges(v.N0);     // band b = output rows [edge[b], edge[b+1])
-    const int nb = (int)edge.size() - 1;
-    std::vector<double> mu;
-    host_means(m, mu);
-    int rc = table_set_means(m, mu.data(), m->s_comp);
-    if (rc) return rc;
-
-    // equally spaced frames of one pinned allocation and no row padding: one 2-D copy per stack and band
-    const ptrdiff_t max_pitch = ((ptrdiff_t)1 << 31) - 1;
-    auto spacing = [&](const std::vector<const float *> &h) -> ptrdiff_t {
-        if (pitch != W || (ptrdiff_t)H * W * (ptrdiff_t)sizeof(float) > max_pitch) return 0;
-        if (Na < 2) return (ptrdiff_t)H * W;
-        const ptrdiff_t d = h[1] - h[0];
-        if (d < (ptrdiff_t)H * W || d * (ptrdiff_t)sizeof(float) > max_pitch) return 0;
-        for (int k = 2; k < Na; k++) if (h[k] - h[k - 1] != d) return 0;
-        return same_allocation(h[0], h[Na - 1] + (size_t)H * W) ? d : 0;
-    };
-    const ptrdiff_t gap_s = spacing(m->h_sam_f), gap_r = spacing(m->h_ref_f);
-    auto upload = [&](float *dst, const std::vector<const float *> &h, ptrdiff_t gap, int y0, int y1) -> cudaError_t {
-        const size_t rb = (size_t)W * sizeof(float);
-        if (gap > 0)
-            return cudaMemcpy2DAsync(dst + (size_t)y0 * pitch, (size_t)H * rb, h[0] + (size_t)y0 * W, (size_t)gap * sizeof(float),
-                                     (size_t)(y1 - y0) * rb, Na, cudaMemcpyHostToDevice, m->s_copy);
-        for (int k = 0; k < Na; k++) {
-            cudaError_t e = cudaMemcpy2DAsync(dst + ((size_t)k * H + y0) * pitch, (size_t)pitch * sizeof(float), h[k] + (size_t)y0 * W, rb,
-                                              rb, (size_t)(y1 - y0), cudaMemcpyHostToDevice, m->s_copy);
-            if (e != cudaSuccess) return e;
-        }
-        return cudaSuccess;
-    };
-
-    std::vector<cudaEvent_t> ev(2 * nb, nullptr);
-    auto fail = [&](int code) {
-        cudaStreamSynchronize(m->s_copy); cudaStreamSynchronize(m->s_comp); cudaStreamSynchronize(m->s_out);
-        for (auto e : ev) if (e) cudaEventDestroy(e);
-        return code;
-    };
-#define ST_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { \
-        umpa_set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #call, cudaGetErrorString(e_)); return fail(UMPA_ERR_CUDA); } } while (0)
-    for (auto &e : ev) ST_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    const bool trace = getenv("UMPA_STREAM_TRACE") != nullptr;     // timeline of the three streams on stderr
-    std::vector<cudaEvent_t> tev;                // trace only: start, then per band: copy, comp, out
-    auto mark = [&](cudaStream_t st) {
-        if (!trace) return;
-        cudaEvent_t e = nullptr;
-        cudaEventCreate(&e);
-        cudaEventRecord(e, st);
-        tev.push_back(e);
-    };
-    if (trace) { cudaStreamSynchronize(m->s_copy); cudaStreamSynchronize(m->s_comp); }
-    mark(m->s_copy);
-    int up_hi = 0, launches = 0;                // rows [0, up_hi) are on the device and centred
-    for (int b = 0; b < nb; b++) {
-        const int r0 = edge[b], r1 = edge[b + 1];
-        const int need = b == nb - 1 ? H : std::min(H, v.off0 + v.step0 * (r1 - 1) + m->padding + 1);
-        const int hi = std::max(up_hi, need);
-        if (hi > up_hi) {
-            ST_CUDA(upload(m->d_sam32, m->h_sam_f, gap_s, up_hi, hi));
-            ST_CUDA(upload(m->d_ref32, m->h_ref_f, gap_r, up_hi, hi));
-        }
-        ST_CUDA(cudaEventRecord(ev[2 * b], m->s_copy));
-        mark(m->s_copy);
-        ST_CUDA(cudaStreamWaitEvent(m->s_comp, ev[2 * b], 0));
-        if ((rc = table_center_rows_inplace(m, up_hi, hi, m->s_comp))) return fail(rc);
-        up_hi = hi;
-        RoiView vb = v;
-        vb.off0 = v.off0 + v.step0 * r0; vb.N0 = r1 - r0;
-        const size_t px0 = (size_t)r0 * v.N1;
-        if (v.abc) vb.abc = v.abc + 3 * px0;
-        if (v.cover) vb.cover = v.cover + px0;
-        const umpa_outputs db = offset_outputs(dev, px0);
-        m->last_launches = 0;
-        if ((rc = match_view(m, vb, db, m->s_comp, true))) return fail(rc);
-        launches += m->last_launches;
-        ST_CUDA(cudaEventRecord(ev[2 * b + 1], m->s_comp));
-        mark(m->s_comp);
-        ST_CUDA(cudaStreamWaitEvent(m->s_out, ev[2 * b + 1], 0));
-        if ((rc = download_outputs(offset_outputs(host, px0), db, (size_t)(r1 - r0) * v.N1, m->s_out))) return fail(rc);
-        mark(m->s_out);
-    }
-    m->last_launches = launches;
-    ST_CUDA(cudaStreamSynchronize(m->s_out));
-    ST_CUDA(cudaStreamSynchronize(m->s_comp));
-    ST_CUDA(cudaStreamSynchronize(m->s_copy));
-#undef ST_CUDA
-    if (trace) {
-        fprintf(stderr, "[umpa stream] float32 frames, %d bands\n", nb);
-        for (int b = 0; b < nb; b++) {
-            float tc = 0.f, tk = 0.f, to = 0.f;
-            cudaEventElapsedTime(&tc, tev[0], tev[1 + 3 * b]);
-            cudaEventElapsedTime(&tk, tev[0], tev[2 + 3 * b]);
-            cudaEventElapsedTime(&to, tev[0], tev[3 + 3 * b]);
-            fprintf(stderr, "[umpa stream] band %2d: uploaded %.2f  computed %.2f  downloaded %.2f ms\n", b, tc, tk, to);
-        }
-        for (auto e : tev) cudaEventDestroy(e);
-    }
-    for (auto e : ev) if (e) cudaEventDestroy(e);
-    m->host_pending = false;
-    m->fp64_missing = true;                     // no FP64 copy on the device: ensure_resident widens one on demand
-    m->stream_bands = nb; m->stream_threads = 0; m->stream_host_rows = 0;
     return UMPA_OK;
 }
 
@@ -1293,7 +1182,7 @@ int umpa_match_host(umpa_model *m, const int32_t roi[6], const double uv0[2], co
 
     // frames still on the host and the table path applies: pipeline upload / kernels / download
     if (m->host_pending && m->path_opt != UMPA_PATH_LAZY && !getenv("UMPA_NO_STREAMING") && table_eligible(m, v, nullptr)) {
-        rc = streamed_match(m, v, d, *out);        // (float32 frames: it picks the plain or the host-staged pipeline)
+        rc = streamed_match(m, v, d, *out);
         record_last(m, m->s_comp);                 // (it returns with its three streams drained)
         return rc;
     }
